@@ -17,6 +17,9 @@ Headline metric: Mpix/s of the 5x5 box filter on image2d<vuchar3> (BASELINE conf
            each with `parity` (checked against the oracle in this run) and a reference-kind CPU figure beside it.
 --impl reference times the reference's own CPU implementation (oracle/_ref = the reference headers compiled with its
 benchmark flags -O3 -march=native -fopenmp; the oracle port only if that library is missing) on the host cores.
+--dump-outputs DIR writes what the timed step computed (see dump_outputs) so that two builds can be compared output for output;
+the inputs are seeded, identical from run to run.
+The bench runs from the tree build() left and writes nothing into it.
 """
 import argparse
 import ctypes as C
@@ -30,11 +33,13 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # no __pycache__ in the tree: it may be read-only
 sys.path.insert(0, ROOT)
 
 WORKLOADS = {"1080p": (1080, 1920), "4k": (2160, 3840), "8k": (4320, 7680)}
 BOX_BYTES_PER_PX = 6.0  # algorithmic: 3 B read + 3 B written per vuchar3 pixel (SURVEY 8d)
 BATCH_1GPU, BATCH_TILED = 128, 32  # resident frame pairs = frames per launch (1080p frames at N = 1, 8K row tiles at N > 1)
+DUMP_BYTES = 48e6  # --dump-outputs budget over all ranks (at most 64 MB)
 
 
 def peaks():
@@ -326,6 +331,20 @@ def passes_for(ms_per_batch, target_ms=5.5):
     return int(max(1, min(512, np.ceil(target_ms / max(ms_per_batch, 1e-3)))))
 
 
+def dump_outputs(out_dir, dst, rank, world):
+    """The filtered frames the timed step left in this rank's output images (its row tile of each frame at N > 1), as float32
+    out_dir/box5x5.npy (box5x5_rank<r>.npy at N > 1) of shape (frames, rows, cols, 3): every row when they fit DUMP_BYTES, else the
+    same number of rows of every frame, drawn per frame from a generator seeded with the rank (sorted)."""
+    os.makedirs(out_dir, exist_ok=True)
+    nrows, ncols = dst[0].nrows, dst[0].ncols
+    keep = int(max(1, min(nrows, DUMP_BYTES / world // (len(dst) * ncols * 3 * 4))))
+    rng = np.random.default_rng(rank)
+    out = np.empty((len(dst), keep, ncols, 3), np.float32)
+    for i, d in enumerate(dst):
+        out[i] = d.download()[np.sort(rng.choice(nrows, keep, replace=False))]
+    np.save(os.path.join(out_dir, "box5x5.npy" if world == 1 else "box5x5_rank%d.npy" % rank), out)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -337,6 +356,7 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--graph", type=int, default=1)
     ap.add_argument("--cpu-budget", type=float, default=12.0, help="seconds of CPU work for the cpu_baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the outputs of the last timed step to DIR/*.npy (float32)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -370,10 +390,8 @@ def main():
         return 0
 
     import torch
-    import __graft_entry__ as g
 
-    g.build(only_if_missing=True)
-    import vpp_b200 as vpp
+    import vpp_b200 as vpp  # raises when build() has not made vpp_b200/lib/libvppb.so
     from vpp_b200 import capi, tiles
     from tests import oracle as orc  # the checker of what was timed (never the thing measured)
 
@@ -478,6 +496,8 @@ def main():
         orc.load(omp=True).vo_box5x5_u8(hs.ptr(), h_.ptr(), 3)
         hd.append(h_.get())
     parity_ok = bool(np.array_equal(dst[0].download(), hd[0]) and np.array_equal(dst[BATCH - 1].download(), hd[1]))
+    if args.dump_outputs:  # every step (timed or the untimed continuation above) writes the same outputs from the same resident inputs
+        dump_outputs(args.dump_outputs, dst, rank, world)
 
     alg_bytes = BOX_BYTES_PER_PX * th * W * BATCH  # per launch, this rank
     us_per_launch = ms_total * 1e3 / (steps * passes)

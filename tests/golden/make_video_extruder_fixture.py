@@ -37,9 +37,9 @@ def eventful_frames(nr=NR, nc=NC, nf=NF, seed=77):
 
 
 def reference_table(frames, nframes, detector_th):
-    from tests.test_oracle_vs_ref import REF_OMP, _load
+    from tests.golden.make_reference_vectors import REF_OMP, load_ref
 
-    ref = _load(REF_OMP)
+    ref = load_ref(REF_OMP)
     ref.vppref_set_num_threads(1)
     nr, nc = frames[0].shape
     hosts = [orc.HostImage(nr, nc, "u8", border=10, aligned=32, data=f, fill_border="mirror") for f in frames[:nframes]]

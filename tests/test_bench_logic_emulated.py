@@ -11,6 +11,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 RUNNER = os.path.join(ROOT, "tests", "emu", "run_bench_emulated.py")
 KEYS = ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype", "data", "config",
@@ -22,8 +24,8 @@ def _run(rows, cols, bench_args, env=None):
                             text=True, cwd=ROOT, env=env or dict(os.environ))
 
 
-def test_bench_single_gpu_control_flow(built):
-    p = _run(48, 400, ["--steps", "3", "--warmup", "3", "--passes", "2", "--no-extras", "--cpu-budget", "0.2"])
+def test_bench_single_gpu_control_flow(built, tmp_path):
+    p = _run(48, 400, ["--steps", "3", "--warmup", "3", "--passes", "2", "--no-extras", "--cpu-budget", "0.2", "--dump-outputs", str(tmp_path)])
     out, err = p.communicate(timeout=900)
     assert p.returncode == 0, err[-3000:]
     line = json.loads(out.strip().splitlines()[-1])
@@ -36,6 +38,18 @@ def test_bench_single_gpu_control_flow(built):
     ef = line["e2e"]["frames_per_e2e_step"]
     assert line["e2e"]["h2d_bytes_per_step"] == ef * 48 * 400 * 3 and line["e2e"]["d2h_bytes_per_step"] == ef * 48 * 400 * 3
     assert line["cpu_baseline"]["kind"] in ("reference", "port") and line["cpu_baseline"]["cores"] >= 1
+    # --dump-outputs: at this size every row of the 128 output frames fits; frame i is the box filter of seeded input i % 4
+    from bench import make_frames
+    from tests import oracle as orc
+
+    assert os.listdir(str(tmp_path)) == ["box5x5.npy"]
+    out = np.load(str(tmp_path / "box5x5.npy"))
+    assert out.dtype == np.float32 and out.shape == (nb, 48, 400, 3)
+    for i, f in enumerate(make_frames(48, 400, 4)):
+        hs = orc.HostImage(48, 400, "vuchar3", border=2, data=f, fill_border="mirror")
+        hd = orc.HostImage(48, 400, "vuchar3")
+        orc.load().vo_box5x5_u8(hs.ptr(), hd.ptr(), 3)
+        assert np.array_equal(out[i::4], np.broadcast_to(hd.get(), out[i::4].shape)), i
 
 
 def test_bench_reference_arm(built):

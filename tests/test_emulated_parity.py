@@ -48,12 +48,16 @@ def vpp(built, request):
         fn.restype, fn.argtypes = res, args
     emu.vppb_emu_set_reverse(1 if request.param == "reversed" else 0)
     emu.vppb_emu_set_shuffle(12345 if request.param == "shuffled" else 0)
+    # ops caches FAST workspaces across calls: a cached buffer must be freed by the library that allocated it and never reach
+    # the other one (emulator buffers are host memory; freeing one with cudaFree leaves an error pending in the CUDA runtime)
+    ops._FAST_CACHE.clear()
     mp = pytest.MonkeyPatch()
     mp.setattr(capi, "lib", emu)
     mp.setattr(ops, "lib", emu)
     yield vpp_b200
     emu.vppb_emu_set_reverse(0)
     emu.vppb_emu_set_shuffle(0)
+    ops._FAST_CACHE.clear()
     gc.collect()  # images allocated by the emulated library must be freed by it
     mp.undo()
     logs = glob.glob(UBSAN_LOG + "*")

@@ -31,10 +31,12 @@ def vpp(built):
     for name, (res, args) in capi.PROTOTYPES.items():
         fn = getattr(emu, name)
         fn.restype, fn.argtypes = res, args
+    ops._FAST_CACHE.clear()  # cached FAST workspaces are freed by the library that allocated them (tests/test_emulated_parity.py)
     mp = pytest.MonkeyPatch()
     mp.setattr(capi, "lib", emu)
     mp.setattr(ops, "lib", emu)
     yield vpp_b200
+    ops._FAST_CACHE.clear()
     gc.collect()
     mp.undo()
 

@@ -1,20 +1,22 @@
 """SURVEY 8(f) N4 on the CPU: the oracle restatements of lbp_transform, local_maxima_filter, fast_detector9_blockwise_rank and the
-oriented LK matcher against the reference's own test vector (tests/lbp.cc) and against the reference's headers compiled in
-oracle/_ref (lbp_transform.hh, fast.hpp:555-575, lk.hh:180-317; blockwise_rank is not instantiable in the reference - see the oracle)."""
-import ctypes as C
-import os
-
+oriented LK matcher against the reference's own test vector (tests/lbp.cc) and against what the reference's headers (lbp_transform.hh,
+fast.hpp:555-575, lk.hh:180-317) computed on the same inputs, stored in tests/golden/reference_n4.npz by
+tests/golden/make_reference_vectors.py (blockwise_rank is not instantiable in the reference - see the oracle)."""
 import numpy as np
 import pytest
 
 from tests import oracle as orc
+from tests import reference_vectors as rv
 from tests import scenes
 from tests.oracle_ops import oracle_grad_pyramid, oracle_pyramid
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(ROOT, "oracle", "_ref", "libvppref.so")
-needs_ref = pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref not built (needs /root/reference)")
-I = C.POINTER(orc.VoImg)
+# stored random examples of the property pins below (drawn as in tests/test_oracle_vs_ref_property.py)
+SPACES = {"lbp": dict(nr=(1, 30), nc=(1, 70), levels=(1, 255), aligned=[1, 4, 16, 128], seed=(0, 2 ** 16)),
+          "lmf": dict(nr=(1, 24), nc=(1, 40), levels=(1, 40), pix=["u8", "i32"], signed=[False, True], seed=(0, 2 ** 16))}
+EXAMPLES = {"lbp": 300, "lmf": 300}
+LBP_SHAPES = [(3, 3), (37, 53), (64, 128), (5, 301)]
+LMF_SHAPES = [(9, 14), (40, 67), (64, 96)]
+ORIENTED_CASES = [(5, 10, 1.0), (7, 21, 0.5), (9, 15, 100.0), (11, 4, 2.0)]
 
 
 @pytest.fixture(scope="module")
@@ -23,12 +25,8 @@ def o(built):
 
 
 @pytest.fixture(scope="module")
-def ref(built):
-    r = C.CDLL(REF)
-    r.vppref_lbp_u8.argtypes = [I, I]
-    r.vppref_local_maxima_filter.argtypes = [I]
-    r.vppref_lk_match_oriented.argtypes = [I, I, I, C.c_int, C.c_float, C.c_int, C.c_float, C.c_float] + [C.c_void_p] * 4 + [C.c_int, C.c_void_p, C.c_void_p]
-    return r
+def G():
+    return rv.load("n4")
 
 
 def test_lbp_known_answer(o):
@@ -40,15 +38,17 @@ def test_lbp_known_answer(o):
     assert out.get()[1, 1] == 0b10101110
 
 
-@needs_ref
-@pytest.mark.parametrize("shape", [(3, 3), (37, 53), (64, 128), (5, 301)])
-def test_lbp_equals_reference(ref, o, shape):
+def lbp_input(shape):
     img = np.random.default_rng(shape[1]).integers(0, 6, shape, dtype=np.uint8) * 40
-    h = orc.HostImage(shape[0], shape[1], "u8", border=1, data=img, fill_border="mirror")
-    a, b = orc.HostImage(shape[0], shape[1], "u8"), orc.HostImage(shape[0], shape[1], "u8")
-    ref.vppref_lbp_u8(h.ptr(), a.ptr())
+    return orc.HostImage(shape[0], shape[1], "u8", border=1, data=img, fill_border="mirror")
+
+
+@pytest.mark.parametrize("shape", LBP_SHAPES)
+def test_lbp_equals_reference(G, o, shape):
+    h = lbp_input(shape)
+    b = orc.HostImage(shape[0], shape[1], "u8")
     o.vo_lbp_u8(h.ptr(), b.ptr())
-    assert np.array_equal(a.get(), b.get()) and len(np.unique(b.get())) > 3
+    assert rv.digest(b.get()) == G["lbp_%dx%d" % shape] and len(np.unique(b.get())) > 3
 
 
 def lmf_scenes(shape, pix, seed):
@@ -65,16 +65,13 @@ def lmf_scenes(shape, pix, seed):
     return [a.astype(np.uint8 if pix == "u8" else np.int32) for a in out]
 
 
-@needs_ref
 @pytest.mark.parametrize("pix", ["u8", "i32"])
-@pytest.mark.parametrize("shape", [(9, 14), (40, 67), (64, 96)])
-def test_local_maxima_filter_serial_equals_reference(ref, o, shape, pix):
+@pytest.mark.parametrize("shape", LMF_SHAPES)
+def test_local_maxima_filter_serial_equals_reference(G, o, shape, pix):
     for i, img in enumerate(lmf_scenes(shape, pix, 3)):
-        a = orc.HostImage(shape[0], shape[1], pix, border=1, data=img, fill_border="value")
         b = orc.HostImage(shape[0], shape[1], pix, border=1, data=img, fill_border="value")
-        ref.vppref_local_maxima_filter(a.ptr())
         o.vo_local_maxima_filter(b.ptr())
-        assert np.array_equal(a.get(True), b.get(True)), (i, pix)
+        assert rv.digest(b.get(True)) == G["lmf_%s_%dx%d_%d" % ((pix,) + shape + (i,))], (i, pix)
         assert (b.get() != img).any() or i == 2
 
 
@@ -92,24 +89,24 @@ def oriented_case(nr, nc, n, seed, ws):
     return f1, f2, np.ascontiguousarray(pts, np.float32), pred, d1, d2
 
 
-@needs_ref
-@pytest.mark.parametrize("ws,max_iter,max_step", [(5, 10, 1.0), (7, 21, 0.5), (9, 15, 100.0), (11, 4, 2.0)])
-def test_oriented_lk_equals_reference(ref, o, ws, max_iter, max_step):
+def oriented_inputs(ws, o):
+    """frames (borders mirror-filled), float Scharr gradient of the first, keypoints, predictions and window directions"""
     nr, nc = 151, 203
     f1, f2, pts, pred, d1, d2 = oriented_case(nr, nc, 300, ws, ws)
-    n = len(pts)
     A = orc.HostImage(nr, nc, "u8", border=3, data=f1, fill_border="mirror")
     B = orc.HostImage(nr, nc, "u8", border=3, data=f2, fill_border="mirror")
-    G = oracle_grad_pyramid([A], "vfloat2", 3, o)[0]
-    fa, ea = np.zeros((n, 2), np.float32), np.zeros(n, np.float32)
+    return A, B, oracle_grad_pyramid([A], "vfloat2", 3, o)[0], pts, pred, d1, d2
+
+
+@pytest.mark.parametrize("ws,max_iter,max_step", ORIENTED_CASES)
+def test_oriented_lk_equals_reference(G, o, ws, max_iter, max_step):
+    A, B, Gr, pts, pred, d1, d2 = oriented_inputs(ws, o)
+    n = len(pts)
     fb, eb = np.zeros((n, 2), np.float32), np.zeros(n, np.float32)
-    ref.vppref_lk_match_oriented(A.ptr(), B.ptr(), G.ptr(), ws, 1e-3, max_iter, 0.01, max_step, pts.ctypes.data, pred.ctypes.data, d1.ctypes.data,
-                                 d2.ctypes.data, n, fa.ctypes.data, ea.ctypes.data)
-    o.vo_lk_match_oriented_u8(A.ptr(), B.ptr(), G.ptr(), 1, ws, 1e-3, max_iter, 0.01, max_step, pts.ctypes.data, pred.ctypes.data, d1.ctypes.data,
+    o.vo_lk_match_oriented_u8(A.ptr(), B.ptr(), Gr.ptr(), 1, ws, 1e-3, max_iter, 0.01, max_step, pts.ctypes.data, pred.ctypes.data, d1.ctypes.data,
                               d2.ctypes.data, n, fb.ctypes.data, eb.ctypes.data)
-    # points whose rotated windows leave the domain use uninitialised as[] / gs[] in the reference (zero here): the first four
-    same = (fa.view(np.int32) == fb.view(np.int32)).all(axis=1) & (ea.view(np.int32) == eb.view(np.int32))
-    assert same[4:].all(), (np.flatnonzero(~same), fa[~same][:4], fb[~same][:4])
+    # points whose rotated windows leave the domain use uninitialised as[] / gs[] in the reference (zero here): the first four are not stored
+    assert rv.digest(fb[4:], eb[4:]) == G["oriented_%d" % ws]
     ok = eb < 1e30
     assert ok.sum() > n // 2 and (np.abs(fb[ok] - np.array([1.3, -0.8])).max(axis=1) < 1.0).mean() > 0.5
 
@@ -144,35 +141,29 @@ def test_blockwise_rank_properties(o):
             assert (np.diff(sc[m]) <= 0).all()
 
 
-# ---- property-based pins (hypothesis, derandomized like tests/test_oracle_vs_ref_property.py): random geometries and value ranges
-from hypothesis import HealthCheck, given, settings  # noqa: E402
-from hypothesis import strategies as st  # noqa: E402
-
-PSET = dict(max_examples=300, deadline=None, derandomize=True, suppress_health_check=[HealthCheck.function_scoped_fixture, HealthCheck.too_slow])
-
-
-@needs_ref
-@settings(**PSET)
-@given(nr=st.integers(1, 30), nc=st.integers(1, 70), levels=st.integers(1, 255), aligned=st.sampled_from([1, 4, 16, 128]), seed=st.integers(0, 2 ** 16))
-def test_lbp_any_geometry(ref, o, nr, nc, levels, aligned, seed):
+# ---- property pins over stored random examples (SPACES above): random geometries and value ranges
+def lbp_any_input(nr, nc, levels, aligned, seed):
     img = np.random.default_rng(seed).integers(0, levels + 1, (nr, nc)).astype(np.uint8)
-    h = orc.HostImage(nr, nc, "u8", border=1, aligned=aligned, data=img, fill_border="value", border_value=seed % 256)
-    a, b = orc.HostImage(nr, nc, "u8", aligned=aligned), orc.HostImage(nr, nc, "u8", aligned=aligned)
-    ref.vppref_lbp_u8(h.ptr(), a.ptr())
-    o.vo_lbp_u8(h.ptr(), b.ptr())
-    assert np.array_equal(a.get(), b.get())
+    return orc.HostImage(nr, nc, "u8", border=1, aligned=aligned, data=img, fill_border="value", border_value=seed % 256)
 
 
-@needs_ref
-@settings(**PSET)
-@given(nr=st.integers(1, 24), nc=st.integers(1, 40), levels=st.integers(1, 40), pix=st.sampled_from(["u8", "i32"]), signed=st.booleans(), seed=st.integers(0, 2 ** 16))
-def test_local_maxima_filter_any_image(ref, o, nr, nc, levels, pix, signed, seed):
-    """few grey levels = many ties and plateaus: the strict comparisons and the in-place order decide everything"""
+def lmf_any_input(nr, nc, levels, pix, signed, seed):
     lo = -levels if (signed and pix == "i32") else 0
     img = np.random.default_rng(seed).integers(lo, levels + 1, (nr, nc)).astype(np.uint8 if pix == "u8" else np.int32)
-    bv = seed % 5
-    a = orc.HostImage(nr, nc, pix, border=1, data=img, fill_border="value", border_value=bv)
-    b = orc.HostImage(nr, nc, pix, border=1, data=img, fill_border="value", border_value=bv)
-    ref.vppref_local_maxima_filter(a.ptr())
-    o.vo_local_maxima_filter(b.ptr())
-    assert np.array_equal(a.get(True), b.get(True))
+    return orc.HostImage(nr, nc, pix, border=1, data=img, fill_border="value", border_value=seed % 5)
+
+
+def test_lbp_any_geometry(G, o):
+    for i, p in rv.cases(SPACES, EXAMPLES, "lbp"):
+        h = lbp_any_input(**p)
+        b = orc.HostImage(p["nr"], p["nc"], "u8", aligned=p["aligned"])
+        o.vo_lbp_u8(h.ptr(), b.ptr())
+        assert rv.digest(b.get()) == G["lbp_digest"][i], p
+
+
+def test_local_maxima_filter_any_image(G, o):
+    """few grey levels = many ties and plateaus: the strict comparisons and the in-place order decide everything"""
+    for i, p in rv.cases(SPACES, EXAMPLES, "lmf"):
+        b = lmf_any_input(**p)
+        o.vo_local_maxima_filter(b.ptr())
+        assert rv.digest(b.get(True)) == G["lmf_digest"][i], p
