@@ -14,8 +14,7 @@ sys.path.insert(0, ROOT)
 VARIANTS = [
     ("default", {}),
     ("tile", {"VPPB_BOX_IMPL": "tile"}),
-    ("stream_lw4", {"VPPB_BOX_LW": "4", "VPPB_BOX_SINGLE": "stream"}),
-    ("stream_lw4_occ", {"VPPB_BOX_LW": "4", "VPPB_BOX_OCC": "1", "VPPB_BOX_SINGLE": "stream"}),
+    ("stream_single", {"VPPB_BOX_SINGLE": "stream"}),
 ]
 
 

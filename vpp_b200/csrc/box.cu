@@ -291,31 +291,42 @@ __global__ void __launch_bounds__(BX_THREADS, BX_TH == 16 ? 4 : 6) k_box5_bytes_
 }
 
 // ------------------------------------------------------------------ streaming kernel (bytes)
-// Every WARP is an independent stream processor: it owns a strip of 32 x 4 LW output bytes (LW words per lane) and
-// walks down a chunk of R output rows.  Lane 0 keeps a ring of STAGES TMA boxes in flight (16 bytes left + strip + 16
-// right, by BS_K = 5 rows; one mbarrier per stage, owned by the warp) - no CTA-wide barrier anywhere, and the pipeline
-// keeps running from one task of the warp into its next one.  Per input row a lane
-//   loads its window from the stage (LDS.64 + LW/4 x LDS.128 + LDS.64: bytes x-8 .. x+4LW+7),
-//   splits the words into packed 16-bit lanes E = (b0,b2), O = (b1,b3) and forms the 5 horizontal taps CS bytes apart
-//     (whole or word-straddling lane pairs, one PRMT each)  ->  H = horizontal 5-sum of the raw row, 2 LW registers,
-//   slides the vertical window in registers: S += H - H(5 rows ago)  (ring of 5 rows, statically indexed because a
-//     stage is exactly 5 rows),
-//   and for every completed window divides by 25 (exact multiply-shift) and stores its bytes (contiguous per warp).
+// The work is cut into UNITS: 128 output bytes of the rows of one row chunk (R rows of one image).  A WARP takes BS_UPW = 4
+// consecutive units in the flattened (image, row chunk, column unit) order - they may lie in different row chunks or images -
+// so a row whose byte width is a multiple of 128 leaves no lane without work.  8 lanes share a unit, each owning BS_LW = 4
+// output words, and the warp walks its units down their chunks in lockstep.  Per stage of BS_K = 5 input rows, lanes 0..3
+// each fetch their unit's 160 x 5 byte TMA box (16 bytes left + 128 + 16 right) into a ring of BS_STAGES stages; the stage
+// mbarrier takes one arrival per unit.  No CTA-wide barrier anywhere, and the pipeline keeps running from one task of the
+// warp into its next one.  Per input row a lane
+//   loads its window from the stage (LDS.64 + LDS.128 + LDS.64: bytes x-8 .. x+23),
+//   splits the words into packed 16-bit lanes O = (b1,b3) (one PRMT) and E = (b0,b2) = w - 256 O (one IMAD),
+//   forms the 5 horizontal taps CS bytes apart (whole or word-straddling lane pairs, one PRMT each) -> H, 8 registers,
+//   slides the vertical window in registers: S += H - H(5 rows ago) (a ring of 5 rows, statically indexed because a stage
+//     is exactly 5 rows),
+//   and for every completed window divides by 25 (exact multiply-shift) and stores its 16 bytes.
 // Horizontal-first means the only data exchanged between lanes is the raw halo, which TMA already put in shared memory:
 // no shared-memory writes, no __syncthreads; one __syncwarp per stage before its buffer is handed back to TMA.
-// The packed-lane additions are split between the ALU pipe (IADD3 / PRMT / LOP3, the busier one) and the FMA pipe
-// (IMAD with a run-time multiplier of 1, which ptxas cannot fold back into an IADD3).
-constexpr int BS_K = 5;  // rows per stage == rows of the vertical window
+// The ALU pipe (PRMT / IADD3 / LOP3) and the FMA pipe (IMAD) each take a warp instruction every other cycle.  The byte split
+// and the divide use IMADs with run-time multipliers (-256, 2^16), which ptxas cannot turn back into ALU instructions; the
+// additions are left to ptxas, which moves some of them to the FMA pipe as IMAD.IADD.  A steady-state row then issues about
+// as many instructions as twice either pipe's share (profiles/r3_box_stream.md).
+// A task is R = 5 m - 4 output rows, exactly m stages.  A stage after the first whose 5 rows all lie inside every unit's
+// chunk, in a warp whose lanes all store whole 16-byte words, runs without any per-row predicate.  The first stage of a task
+// (input rows 0..3 complete no window), a stage past the last row of an image and a warp with lanes at the right edge of the
+// image take the checked path.
+constexpr int BS_K = 5;            // rows per stage == rows of the vertical window
 constexpr int BS_MAX_BATCH = 128;  // images per launch of the streaming kernel (their tensor maps travel in the 32 KB kernel parameter space)
-template <int LW, int OCC = 0> struct BoxStreamCfg {  // OCC = 1: one more CTA per SM (fewer registers, one stage less)
-  static constexpr int STRIP = 32 * 4 * LW;          // output bytes per warp row
-  static constexpr int BOXW = STRIP + 32;            // bytes per box row
-  static constexpr int STAGE_BYTES = ((BS_K * BOXW + 127) / 128) * 128;
-  static constexpr int WARPS = 4;
-  static constexpr int STAGES = (LW == 4 ? 4 : 3) - OCC;
-  static constexpr int CTAS_PER_SM = (LW == 4 ? 4 : 3) + OCC;
-  static constexpr int SMEM = WARPS * STAGES * STAGE_BYTES + WARPS * STAGES * 8;
-};
+constexpr int BS_LW = 4;                                              // output words per lane
+constexpr int BS_UNIT = 128;                                          // output bytes of a unit row
+constexpr int BS_LPU = BS_UNIT / (4 * BS_LW);                         // lanes per unit (8)
+constexpr int BS_UPW = 32 / BS_LPU;                                   // units per warp (4)
+constexpr int BS_BOXW = BS_UNIT + 32;                                 // bytes per box row (160)
+constexpr int BS_UNIT_BYTES = ((BS_K * BS_BOXW + 127) / 128) * 128;   // one unit's box in a stage (TMA destinations are 128-byte aligned)
+constexpr int BS_STAGE_BYTES = BS_UPW * BS_UNIT_BYTES;
+constexpr int BS_WARPS = 4;
+constexpr int BS_STAGES = 3;
+constexpr int BS_CTAS_PER_SM = 4;  // 16 warps per SM: at most 128 registers per thread
+constexpr int BS_SMEM = BS_WARPS * BS_STAGES * (BS_STAGE_BYTES + 8);
 
 template <int NB>
 struct BoxStream {
@@ -326,7 +337,7 @@ struct BoxStream {
   const unsigned char* in_base[NB];
   const unsigned char* up_base[NB];
   const unsigned char* dn_base[NB];
-  int nimg, out_pitch, nrows, rowbytes, strips, chunks, R, groups, vec_store, total;
+  int out_pitch, nrows, rowbytes, ucols, chunks, R, groups, vec_store, units, tasks;
   int in_pitch, row_room;   // row_room: addressable bytes of a row from pixel (0,0) to the end of its pitch
   uint32_t one;
 };
@@ -341,21 +352,56 @@ __device__ __forceinline__ uint32_t box_div_pack_hi(uint32_t se, uint32_t so, ui
   return __byte_perm(lo, hi, 0x5410);
 }
 
-// the rare partial store of a lane that straddles the right edge of the image (kept out of the hot loop)
-template <int LW>
+// the partial store of a lane that straddles the right edge of the image, or of an unaligned output (kept out of the hot loop)
 __device__ __noinline__ void box_store_partial(unsigned char* d, const uint32_t* ow, int nbytes) {
   for (int k = 0; k < nbytes; k++) d[k] = (unsigned char)(ow[k >> 2] >> ((k & 3) * 8));
 }
 
-// A stage that straddles a row-tile seam: row by row, each from the tile that owns it - the halo rows come straight from
-// the neighbour's (peer GPU's) memory as 1-D bulk copies, so the transfer is part of the kernel's own load pipeline.
-template <int LW, int NB>
-__device__ __noinline__ void box_stage_from_tiles(const BoxStream<NB>& p, unsigned char* stage, uint64_t* bar, int img, int strip, int ty) {
-  typedef BoxStreamCfg<LW> Cfg;
+// One input row of a lane: rp = its window in the stage (8 bytes left of its first output byte).  Leaves the horizontal
+// 5-sums of the row in (rE, rO) (the ring slot of this row, which held the row 5 rows up) and slides (SE, SO) by them.
+template <int CS>
+__device__ __forceinline__ void box_stream_row(const unsigned char* rp, uint32_t (&rE)[BS_LW], uint32_t (&rO)[BS_LW], uint32_t (&SE)[BS_LW],
+                                               uint32_t (&SO)[BS_LW], uint32_t m256) {
+  constexpr int NW = BS_LW + 4;  // words of a lane's window: 2 left + BS_LW own + 2 right
+  static_assert(BS_LW == 4, "the window is loaded as 2 + 4 + 2 words");
+  const uint2 wl = *reinterpret_cast<const uint2*>(rp);
+  const uint4 wm = *reinterpret_cast<const uint4*>(rp + 8);
+  const uint2 wr = *reinterpret_cast<const uint2*>(rp + 24);
+  const uint32_t w[NW] = {wl.x, wl.y, wm.x, wm.y, wm.z, wm.w, wr.x, wr.y};
+  uint32_t E[NW], O[NW], XE[NW - 1], XO[NW - 1];
+#pragma unroll
+  for (int i = 0; i < NW; i++) {
+    O[i] = __byte_perm(w[i], 0u, 0x4341);  // (b1, b3)
+    E[i] = fadd_u32(O[i], m256, w[i]);     // (b0, b2) = w - 256 O, on the FMA pipe
+  }
+#pragma unroll
+  for (int i = 0; i < NW - 1; i++) { XE[i] = __byte_perm(E[i], E[i + 1], 0x5432); XO[i] = __byte_perm(O[i], O[i + 1], 0x5432); }
+#pragma unroll
+  for (int q = 0; q < BS_LW; q++) {
+    const int i = q + 2;
+    uint32_t he, ho;
+    if (CS == 3) {  // lanes (x, x+2): taps x-6, x-3, x, x+3, x+6; lanes (x+1, x+3) likewise
+      he = XE[i + 1] + XO[i] + XE[i - 2] + O[i - 1] + E[i];
+      ho = XO[i + 1] + E[i + 1] + XO[i - 2] + XE[i - 1] + O[i];
+    } else {        // CS == 1: taps x-2 .. x+2
+      he = XE[i] + O[i] + XE[i - 1] + XO[i - 1] + E[i];
+      ho = XO[i] + XE[i] + XO[i - 1] + E[i] + O[i];
+    }
+    SE[q] = SE[q] + he - rE[q];  // one IADD3 with a negated operand
+    SO[q] = SO[q] + ho - rO[q];
+    rE[q] = he;
+    rO[q] = ho;
+  }
+}
+
+// A stage that straddles a row-tile seam, for one unit: row by row, each from the tile that owns it - the halo rows come
+// straight from the neighbour's (peer GPU's) memory as 1-D bulk copies, so the transfer is part of the kernel's own load pipeline.
+template <int NB>
+__device__ __noinline__ void box_stage_from_tiles(const BoxStream<NB>& p, unsigned char* dst, uint64_t* bar, int img, int ucol, int ty) {
   const unsigned char* up = p.up_base[img];
   const unsigned char* dn = p.dn_base[img];
-  const int xoff = strip * Cfg::STRIP - 16;
-  const int len = min(Cfg::BOXW, p.row_room - xoff);
+  const int xoff = ucol * BS_UNIT - 16;
+  const int len = min(BS_BOXW, p.row_room - xoff);
   int rows = 0;
   for (int i = 0; i < BS_K; i++) rows += (ty + i - 2 <= p.nrows + 1) ? 1 : 0;
   mbar_arrive_expect_tx(bar, rows * len);
@@ -365,154 +411,136 @@ __device__ __noinline__ void box_stage_from_tiles(const BoxStream<NB>& p, unsign
     const unsigned char* src = (v < 0 && up) ? up + (long long)(p.nrows + v) * p.in_pitch
                              : (v >= p.nrows && dn) ? dn + (long long)(v - p.nrows) * p.in_pitch
                                                     : p.in_base[img] + (long long)v * p.in_pitch;
-    tma_load_1d(stage + i * Cfg::BOXW, src + xoff, len, bar);
+    tma_load_1d(dst + i * BS_BOXW, src + xoff, len, bar);
   }
 }
 
-template <int CS, int LW, int BAL, int NB, int OCC>
-__global__ void __launch_bounds__(BoxStreamCfg<LW, OCC>::WARPS * 32, BoxStreamCfg<LW, OCC>::CTAS_PER_SM) k_box5_stream(const __grid_constant__ BoxStream<NB> p) {
-  typedef BoxStreamCfg<LW, OCC> Cfg;
-  constexpr int NW = LW + 4;  // words of a lane's window: 2 left + LW own + 2 right
+template <int CS, int NB>
+__global__ void __launch_bounds__(BS_WARPS * 32, BS_CTAS_PER_SM) k_box5_stream(const __grid_constant__ BoxStream<NB> p) {
   extern __shared__ __align__(128) unsigned char smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  unsigned char* ring = smem + warp * (Cfg::STAGES * Cfg::STAGE_BYTES);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::WARPS * Cfg::STAGES * Cfg::STAGE_BYTES) + warp * Cfg::STAGES;
-  const int gw = blockIdx.x * Cfg::WARPS + warp, nw = gridDim.x * Cfg::WARPS;
-  const int per_img = p.strips * p.chunks;
-  const uint32_t one = p.one, minus_one = 0u - p.one, shl16 = p.one << 16;
+  unsigned char* ring = smem + warp * (BS_STAGES * BS_STAGE_BYTES);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + BS_WARPS * BS_STAGES * BS_STAGE_BYTES) + warp * BS_STAGES;
+  const int gw = blockIdx.x * BS_WARPS + warp, nw = gridDim.x * BS_WARPS;
+  const int per_img = p.chunks * p.ucols;
+  const uint32_t m256 = 0u - (p.one << 8), shl16 = p.one << 16;  // -256 and 2^16, unknown to ptxas: the multiplies stay IMADs
 
   grid_launch_dependents();  // the next kernel of the stream may be scheduled while this one drains (it waits before it reads)
   if (lane == 0) {
 #pragma unroll
-    for (int s = 0; s < Cfg::STAGES; s++) mbar_init(&bars[s], 1);
+    for (int s = 0; s < BS_STAGES; s++) mbar_init(&bars[s], BS_UPW);  // one arrival per unit
     fence_barrier_init();
   }
   __syncwarp();
   grid_dependency_wait();    // launched programmatically: everything above overlapped the previous kernel's tail; its writes are visible now
 
-  // producer cursor (meaningful in lane 0 only): the next stage to fetch is rows [py, py + 5) of tensor map pmap at element
-  // column px; pleft stages remain in the current task.  A task is decoded once (two divisions), a stage costs a handful of
-  // instructions; only stages that straddle a row-tile seam take the (out-of-line) row-by-row path.
-  int ptask = gw - nw, pslot = 0, pimg = 0, pstrip = 0, py = 0, pleft = 0;
-  bool pseam = false;
+  // producer cursor of lanes 0 .. BS_UPW - 1 (lane = the unit of the warp's task it fetches): the next stage is rows
+  // [py, py + 5) of tensor map pimg at unit column pcol; pleft stages remain in the current task (the same in every lane).
+  // A task is decoded once (two divisions); only stages that straddle a row-tile seam take the (out-of-line) row-by-row path.
+  int ptask = gw - nw, pslot = 0, pimg = 0, pcol = 0, py = 0, pleft = 0;
+  bool pvalid = false, pseam = false;
   auto produce = [&]() {
     if (pleft == 0) {
       ptask += nw;
-      if (ptask < p.total) {
-        pimg = ptask / per_img;
-        const int rem = ptask - pimg * per_img;
-        const int chunk = rem / p.strips;
-        pstrip = rem - chunk * p.strips;
+      if (ptask < p.tasks) {
+        const int u = ptask * BS_UPW + lane;
+        pvalid = u < p.units;  // the last task of a launch may hold fewer units
+        int chunk = 0;
+        if (pvalid) {
+          pimg = u / per_img;
+          const int rem = u - pimg * per_img;
+          chunk = rem / p.ucols;
+          pcol = rem - chunk * p.ucols;
+        }
         py = chunk * p.R;
         pleft = p.groups;
-        pseam = (p.up_base[pimg] && py < 2) || (p.dn_base[pimg] && py + p.groups * BS_K > p.nrows + 2);
+        pseam = pvalid && ((p.up_base[pimg] && py < 2) || (p.dn_base[pimg] && py + p.groups * BS_K > p.nrows + 2));
       }
     }
     if (pleft > 0) {
-      if (pseam && ((p.up_base[pimg] && py < 2) || (p.dn_base[pimg] && py + BS_K > p.nrows + 2)))
-        box_stage_from_tiles<LW, NB>(p, ring + pslot * Cfg::STAGE_BYTES, &bars[pslot], pimg, pstrip, py);
+      unsigned char* dst = ring + pslot * BS_STAGE_BYTES + lane * BS_UNIT_BYTES;
+      if (!pvalid)
+        mbar_arrive(&bars[pslot]);
+      else if (pseam && ((p.up_base[pimg] && py < 2) || (p.dn_base[pimg] && py + BS_K > p.nrows + 2)))
+        box_stage_from_tiles<NB>(p, dst, &bars[pslot], pimg, pcol, py);
       else {
-        mbar_arrive_expect_tx(&bars[pslot], BS_K * Cfg::BOXW);
+        mbar_arrive_expect_tx(&bars[pslot], BS_K * BS_BOXW);
         // tensor origin = 16 bytes left of x = 0 and 2 rows above y = 0; 8-byte elements (x coordinate * 8 is a multiple of 16)
-        tma_load_2d(ring + pslot * Cfg::STAGE_BYTES, &p.maps[pimg], pstrip * (Cfg::STRIP / 8), py, &bars[pslot]);
+        tma_load_2d(dst, &p.maps[pimg], pcol * (BS_UNIT / 8), py, &bars[pslot]);
       }
       py += BS_K;
       pleft--;
     }
-    pslot = (pslot + 1 == Cfg::STAGES) ? 0 : pslot + 1;
+    pslot = (pslot + 1 == BS_STAGES) ? 0 : pslot + 1;
   };
-  if (lane == 0) {
+  if (lane < BS_UPW) {
 #pragma unroll 1
-    for (int s = 0; s < Cfg::STAGES; s++) produce();
+    for (int s = 0; s < BS_STAGES; s++) produce();
   }
 
+  const int lane_off = (lane / BS_LPU) * BS_UNIT_BYTES + (lane % BS_LPU) * (4 * BS_LW) + 8;  // the lane's window in a stage
   int cslot = 0;
   uint32_t parity = 0;
-  for (int task = gw; task < p.total; task += nw) {
-    const int img = task / per_img, rem = task - img * per_img;
-    const int chunk = rem / p.strips, strip = rem - chunk * p.strips;
-    const int x = strip * Cfg::STRIP + lane * (4 * LW);
-    const int y0 = chunk * p.R, yend = min(y0 + p.R, p.nrows);
-    unsigned char* dst = p.out_base[img] + (long long)y0 * p.out_pitch + x;
-    const int nbytes = min(4 * LW, p.rowbytes - x);  // <= 0: this lane is right of the image
-    const bool full = nbytes == 4 * LW && p.vec_store;
-
-    uint32_t rE[BS_K][LW], rO[BS_K][LW], SE[LW], SO[LW];
+  for (int task = gw; task < p.tasks; task += nw) {
+    const int u = task * BS_UPW + lane / BS_LPU;
+    int img = 0, y0 = 0, x = 0, rows = p.R, nbytes = 0;  // nbytes <= 0: the lane is right of the image or its unit is past the last
+    if (u < p.units) {
+      img = u / per_img;
+      const int rem = u - img * per_img;
+      const int chunk = rem / p.ucols;
+      x = (rem - chunk * p.ucols) * BS_UNIT + (lane % BS_LPU) * (4 * BS_LW);
+      y0 = chunk * p.R;
+      rows = min(p.R, p.nrows - y0);
+      nbytes = min(4 * BS_LW, p.rowbytes - x);
+    }
+    const bool full = nbytes == 4 * BS_LW && p.vec_store;
+    const bool clean = __all_sync(0xffffffffu, full);
+    int min_rows = rows;  // the fewest output rows of the warp's units
 #pragma unroll
-    for (int q = 0; q < LW; q++) {
+    for (int o = 16; o > 0; o >>= 1) min_rows = min(min_rows, __shfl_xor_sync(0xffffffffu, min_rows, o));
+
+    uint32_t rE[BS_K][BS_LW], rO[BS_K][BS_LW], SE[BS_LW], SO[BS_LW];
+#pragma unroll
+    for (int q = 0; q < BS_LW; q++) {
       SE[q] = 0; SO[q] = 0;
 #pragma unroll
       for (int j = 0; j < BS_K; j++) { rE[j][q] = 0; rO[j][q] = 0; }
     }
 
-    unsigned char* drow = dst - 4LL * p.out_pitch;  // where the row completed by input row 0 would go; advanced once per input row
+    // input row t of the task completes output row y0 + t - 4: drow is advanced once per input row, before its store
+    unsigned char* drow = p.out_base[img] + (long long)(y0 - 5) * p.out_pitch + x;
+    const long long pitch = p.out_pitch;
     for (int g = 0; g < p.groups; g++) {
       mbar_wait(&bars[cslot], parity);
-      const unsigned char* st = ring + cslot * Cfg::STAGE_BYTES + lane * (4 * LW);
+      const unsigned char* st = ring + cslot * BS_STAGE_BYTES + lane_off;
+      if (clean && g > 0 && BS_K * g < min_rows) {  // steady state: 5 rows of load, compute, store
 #pragma unroll
-      for (int j = 0; j < BS_K; j++) {
-        const unsigned char* rp = st + j * Cfg::BOXW;
-        uint32_t w[NW];
-        {
-          const uint2 wl = *reinterpret_cast<const uint2*>(rp + 8);
-          w[0] = wl.x; w[1] = wl.y;
-#pragma unroll
-          for (int v = 0; v < LW / 4; v++) {
-            const uint4 wm = *reinterpret_cast<const uint4*>(rp + 16 + 16 * v);
-            w[2 + 4 * v] = wm.x; w[3 + 4 * v] = wm.y; w[4 + 4 * v] = wm.z; w[5 + 4 * v] = wm.w;
-          }
-          const uint2 wr = *reinterpret_cast<const uint2*>(rp + 16 + 4 * LW);
-          w[NW - 2] = wr.x; w[NW - 1] = wr.y;
+        for (int j = 0; j < BS_K; j++) {
+          box_stream_row<CS>(st + j * BS_BOXW, rE[j], rO[j], SE, SO, m256);
+          drow += pitch;
+          *reinterpret_cast<uint4*>(drow) = make_uint4(box_div_pack_hi(SE[0], SO[0], shl16), box_div_pack_hi(SE[1], SO[1], shl16),
+                                                       box_div_pack_hi(SE[2], SO[2], shl16), box_div_pack_hi(SE[3], SO[3], shl16));
         }
-        uint32_t E[NW], O[NW], XE[NW - 1], XO[NW - 1];
+      } else {
 #pragma unroll
-        for (int i = 0; i < NW; i++) { E[i] = w[i] & 0x00FF00FFu; O[i] = __byte_perm(w[i], 0u, 0x4341); }
+        for (int j = 0; j < BS_K; j++) {
+          box_stream_row<CS>(st + j * BS_BOXW, rE[j], rO[j], SE, SO, m256);
+          drow += pitch;
+          const int t = BS_K * g + j;  // input row of the task (0 = image row y0 - 2)
+          if (t >= 4 && t - 4 < rows && nbytes > 0) {
+            uint32_t ow[BS_LW];
 #pragma unroll
-        for (int i = 0; i < NW - 1; i++) { XE[i] = __byte_perm(E[i], E[i + 1], 0x5432); XO[i] = __byte_perm(O[i], O[i + 1], 0x5432); }
-#pragma unroll
-        for (int q = 0; q < LW; q++) {
-          const int i = q + 2;
-          uint32_t he, ho;
-          if (CS == 3) {  // lanes (x, x+2): taps x-6, x-3, x, x+3, x+6; lanes (x+1, x+3) likewise
-            he = XE[i + 1] + XO[i] + XE[i - 2] + O[i - 1] + E[i];
-            ho = XO[i + 1] + E[i + 1] + XO[i - 2] + XE[i - 1] + O[i];
-          } else {        // CS == 1: taps x-2 .. x+2
-            he = XE[i] + O[i] + XE[i - 1] + XO[i - 1] + E[i];
-            ho = XO[i] + XE[i] + XO[i - 1] + E[i] + O[i];
-          }
-          if (BAL) {  // S += H - H(5 rows ago) on the FMA pipe (two IMAD)
-            const uint32_t te = fadd_u32(rE[j][q], minus_one, SE[q]), to = fadd_u32(rO[j][q], minus_one, SO[q]);
-            SE[q] = fadd_u32(he, one, te);
-            SO[q] = fadd_u32(ho, one, to);
-          } else {    // one IADD3 with a negated operand
-            SE[q] = SE[q] + he - rE[j][q];
-            SO[q] = SO[q] + ho - rO[j][q];
-          }
-          rE[j][q] = he;
-          rO[j][q] = ho;
-        }
-        const int row = g * BS_K + j;  // input row of the task (0 = image row y0 - 2)
-        if (j > 0 || g > 0) drow += p.out_pitch;
-        if (row >= 4) {
-          const int y = y0 + row - 4;
-          if (y < yend && nbytes > 0) {
-            uint32_t ow[LW];
-#pragma unroll
-            for (int q = 0; q < LW; q++) ow[q] = BAL ? box_div_pack_hi(SE[q], SO[q], shl16) : box_div_pack(SE[q], SO[q]);
-            unsigned char* d = drow;
-            if (full) {
-#pragma unroll
-              for (int v = 0; v < LW / 4; v++)
-                *reinterpret_cast<uint4*>(d + 16 * v) = make_uint4(ow[4 * v], ow[4 * v + 1], ow[4 * v + 2], ow[4 * v + 3]);
-            } else {
-              box_store_partial<LW>(d, ow, nbytes);
-            }
+            for (int q = 0; q < BS_LW; q++) ow[q] = box_div_pack_hi(SE[q], SO[q], shl16);
+            if (full)
+              *reinterpret_cast<uint4*>(drow) = make_uint4(ow[0], ow[1], ow[2], ow[3]);
+            else
+              box_store_partial(drow, ow, nbytes);
           }
         }
       }
       __syncwarp();  // every lane is done reading the stage before TMA refills it
-      if (lane == 0) produce();
-      if (++cslot == Cfg::STAGES) { cslot = 0; parity ^= 1; }
+      if (lane < BS_UPW) produce();
+      if (++cslot == BS_STAGES) { cslot = 0; parity ^= 1; }
     }
   }
 }
@@ -560,7 +588,7 @@ static bool box_use_stream() {
 
 // Rows per task: R = 5 m - 4 (a task then reads exactly m stages).  Small R = more tasks (parallelism for a single
 // frame) but 4 extra input rows per task; pick the R with the smallest makespan estimate over the resident warps.
-static int box_stream_rows(long long strips_x_imgs, int nrows, int warps_per_sm, int* chunks_out) {
+static int box_stream_rows(long long units_x_imgs, int nrows, int warps_per_sm, int* chunks_out) {
   static int forced = -1;
   if (forced < 0) {
     const char* e = getenv("VPPB_BOX_R");
@@ -572,7 +600,7 @@ static int box_stream_rows(long long strips_x_imgs, int nrows, int warps_per_sm,
   for (int m = 4; m <= 26; m++) {
     const int r = 5 * m - 4;
     if (forced > 0 && r != forced) continue;
-    const long long chunks = (nrows + r - 1) / r, tasks = chunks * strips_x_imgs;
+    const long long chunks = (nrows + r - 1) / r, tasks = (chunks * units_x_imgs + BS_UPW - 1) / BS_UPW;
     const long long waves = (tasks + warps - 1) / warps;
     // per task: m stages of 5 rows + ~2 stages of pipeline fill when the warp starts; a wave costs its slowest warp
     const double cost = (double)waves * (5.0 * m + 2.0) + 10.0;
@@ -582,37 +610,36 @@ static int box_stream_rows(long long strips_x_imgs, int nrows, int warps_per_sm,
   return best_r;
 }
 
-// n equally shaped, TMA-eligible images (n <= BX_MAX_BATCH) in one launch of the streaming kernel
-template <int CS, int LW, int BAL, int NB, int OCC>
-static int box5_stream_launch_occ(const vppb_img* ins, const vppb_img* ups, const vppb_img* dns, const vppb_img* outs, int n, cudaStream_t st, const char* name) {
-  typedef BoxStreamCfg<LW, OCC> Cfg;
+// n equally shaped, TMA-eligible images (n <= NB) in one launch of the streaming kernel
+template <int CS, int NB>
+static int box5_stream_launch_nb(const vppb_img* ins, const vppb_img* ups, const vppb_img* dns, const vppb_img* outs, int n, cudaStream_t st, const char* name) {
   const int rowbytes = ins[0].ncols * CS, nrows = ins[0].nrows;
   static std::atomic<unsigned long long> attr_done{0};
   int dev = 0;
   VPPB_CUDA(cudaGetDevice(&dev));
   const unsigned long long bit = 1ULL << (dev & 63);
   if (!(attr_done.load(std::memory_order_acquire) & bit)) {
-    VPPB_CUDA(cudaFuncSetAttribute(k_box5_stream<CS, LW, BAL, NB, OCC>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM));
+    VPPB_CUDA(cudaFuncSetAttribute(k_box5_stream<CS, NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, BS_SMEM));
     attr_done.fetch_or(bit, std::memory_order_release);
   }
   BoxStream<NB> p;
   memset(&p, 0, sizeof(p));
-  p.nimg = n;
   p.out_pitch = outs[0].pitch;
   p.nrows = nrows;
   p.rowbytes = rowbytes;
-  p.strips = (rowbytes + Cfg::STRIP - 1) / Cfg::STRIP;
-  p.R = box_stream_rows((long long)p.strips * n, nrows, Cfg::WARPS * Cfg::CTAS_PER_SM, &p.chunks);
-  p.groups = (p.R + 4 + BS_K - 1) / BS_K;
+  p.ucols = (rowbytes + BS_UNIT - 1) / BS_UNIT;
+  p.R = box_stream_rows((long long)p.ucols * n, nrows, BS_WARPS * BS_CTAS_PER_SM, &p.chunks);
+  p.groups = (p.R + 4) / BS_K;
   p.vec_store = (((uintptr_t)outs[0].base % 16) == 0 && (outs[0].pitch % 16) == 0) ? 1 : 0;
-  p.total = n * p.strips * p.chunks;
+  p.units = n * p.chunks * p.ucols;
+  p.tasks = (p.units + BS_UPW - 1) / BS_UPW;
   p.one = 1u;
   const uint64_t width_el = ((uint64_t)rowbytes + 32 + 7) / 8;
   for (int k = 0; k < n; k++) {
     const vppb_img* in = &ins[k];
     unsigned char* origin = static_cast<unsigned char*>(in->base) - 2LL * in->pitch - 16;
     int rc = encode_tensor_map_2d(&p.maps[k], origin, CU_TENSOR_MAP_DATA_TYPE_UINT64, 8, width_el, (uint64_t)nrows + 4, (uint64_t)in->pitch,
-                                  Cfg::BOXW / 8, BS_K);
+                                  BS_BOXW / 8, BS_K);
     if (rc) return rc;
     p.out_base[k] = static_cast<unsigned char*>(outs[k].base);
     p.in_base[k] = static_cast<const unsigned char*>(in->base);
@@ -625,47 +652,20 @@ static int box5_stream_launch_occ(const vppb_img* ins, const vppb_img* ups, cons
     p.in_pitch = ins[0].pitch;
     p.row_room = ins[0].pitch - (int)bs;
   }
-  const int ctas = (p.total + Cfg::WARPS - 1) / Cfg::WARPS, resident = sm_count() * Cfg::CTAS_PER_SM;
-  VPPB_CUDA(launch_dependent(k_box5_stream<CS, LW, BAL, NB, OCC>, ctas < resident ? ctas : resident, Cfg::WARPS * 32, Cfg::SMEM, st, p));
+  const int ctas = (p.tasks + BS_WARPS - 1) / BS_WARPS, resident = sm_count() * BS_CTAS_PER_SM;
+  VPPB_CUDA(launch_dependent(k_box5_stream<CS, NB>, ctas < resident ? ctas : resident, BS_WARPS * 32, BS_SMEM, st, p));
   VPPB_LAUNCH_CHECK(name);
   return VPPB_OK;
 }
 
-template <int CS, int LW, int BAL, int NB>
-static int box5_stream_launch_nb(const vppb_img* ins, const vppb_img* ups, const vppb_img* dns, const vppb_img* outs, int n, cudaStream_t st, const char* name) {
-  static int occ = -1;
-  if (occ < 0) {
-    const char* e = getenv("VPPB_BOX_OCC");
-    occ = e ? atoi(e) : 0;
-  }
-  if (occ == 1) return box5_stream_launch_occ<CS, LW, BAL, NB, 1>(ins, ups, dns, outs, n, st, name);
-  return box5_stream_launch_occ<CS, LW, BAL, NB, 0>(ins, ups, dns, outs, n, st, name);
-}
-
 // the kernel parameters carry one tensor map per image: a single image travels with a 1-entry block (launching a kernel
-// with kilobytes of parameters costs microseconds), batches with 32
-template <int CS, int LW, int BAL>
-static int box5_stream_launch_lw(const vppb_img* ins, const vppb_img* ups, const vppb_img* dns, const vppb_img* outs, int n, cudaStream_t st, const char* name) {
-  if (n == 1) return box5_stream_launch_nb<CS, LW, BAL, 1>(ins, ups, dns, outs, n, st, name);
-  if (n <= 4) return box5_stream_launch_nb<CS, LW, BAL, 4>(ins, ups, dns, outs, n, st, name);
-  if (n <= 32) return box5_stream_launch_nb<CS, LW, BAL, 32>(ins, ups, dns, outs, n, st, name);
-  return box5_stream_launch_nb<CS, LW, BAL, BS_MAX_BATCH>(ins, ups, dns, outs, n, st, name);
-}
-
+// with kilobytes of parameters costs microseconds), batches with up to 128
 template <int CS>
 static int box5_stream_launch(const vppb_img* ins, const vppb_img* ups, const vppb_img* dns, const vppb_img* outs, int n, cudaStream_t st, const char* name) {
-  static int lw = -1;
-  if (lw < 0) {
-    const char* e = getenv("VPPB_BOX_LW");
-    lw = e ? atoi(e) : 4;
-  }
-  static int bal = -1;
-  if (bal < 0) {
-    const char* e = getenv("VPPB_BOX_BAL");
-    bal = e ? atoi(e) : 0;
-  }
-  if (lw == 8) return bal ? box5_stream_launch_lw<CS, 8, 1>(ins, ups, dns, outs, n, st, name) : box5_stream_launch_lw<CS, 8, 0>(ins, ups, dns, outs, n, st, name);
-  return bal ? box5_stream_launch_lw<CS, 4, 1>(ins, ups, dns, outs, n, st, name) : box5_stream_launch_lw<CS, 4, 0>(ins, ups, dns, outs, n, st, name);
+  if (n == 1) return box5_stream_launch_nb<CS, 1>(ins, ups, dns, outs, n, st, name);
+  if (n <= 4) return box5_stream_launch_nb<CS, 4>(ins, ups, dns, outs, n, st, name);
+  if (n <= 32) return box5_stream_launch_nb<CS, 32>(ins, ups, dns, outs, n, st, name);
+  return box5_stream_launch_nb<CS, BS_MAX_BATCH>(ins, ups, dns, outs, n, st, name);
 }
 
 template <int CS>
